@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the one hot path: HC path tracking of the trifocal_2op1p_30x30 RANSAC round.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--hyp H] [--abort]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--hyp H] [--abort] [--dump-outputs DIR]
 
 One "step" = one RANSAC round: H hypotheses x 312 homotopy paths tracked in one launch per GPU
 (BASELINE.json configs[1]: the full default run — H = 100 = NUM_OF_RANSAC_ITERATIONS, 80 max steps, 3 corrections,
@@ -288,6 +288,35 @@ def _events(torch, n):
     return [torch.cuda.Event(enable_timing=True) for _ in range(n)]
 
 
+DUMP_BYTES = 63 * 1000 * 1000      # per-path arrays of all ranks together; leaves room under 64 MB for the pose record and .npy headers
+
+
+def dump_outputs(out_dir, rank, world, tracks, conv, inf, stats, support, rec):
+    """What the last timed step handed its caller, as DIR/<name>.npy (float32 / float64, values exact): per path the end point
+    (re, im of the 31 entries), converged / infinity flags, the step counters and, when scored, the (inliers21, inliers31) support;
+    and the round's selected pose record.  Inputs are seeded, so two builds can be compared file for file.  With N GPUs every rank
+    writes its own shard as <name>_rank<k>.npy and rank 0 alone the pose record, which all ranks share.  Above DUMP_BYTES / N per rank
+    the per-path arrays are a fixed (seed 0) sample of the rank's paths, in path order; path_index holds the path ids either way."""
+    n = tracks.shape[0]
+    per_path = 31 * 2 * 4 + 4 + 4 + stats.shape[1] * 8 + 8 + (2 * 4 if support is not None else 0)
+    keep = DUMP_BYTES // world // per_path
+    idx = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    arrays = {"path_index": idx.astype(np.float64),
+              "tracks": np.stack([tracks[idx].real, tracks[idx].imag], -1).astype(np.float32),
+              "converged": conv[idx].astype(np.float32), "infinity": inf[idx].astype(np.float32),
+              "stats": stats[idx].astype(np.float64)}
+    if support is not None:
+        arrays["support"] = support[idx].astype(np.float32)
+    suffix = "" if world == 1 else "_rank%d" % rank
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+    if rank == 0:
+        pose = [rec["found"], rec["inliers21"], rec["inliers31"], rec["n_candidates"], rec["abort_flag"], rec["rank"], rec["path_id"]]
+        np.save(os.path.join(out_dir, "round_pose.npy"), np.concatenate([np.array(pose, np.float64), rec["R21"].reshape(-1), rec["t21"],
+                                                                        rec["R31"].reshape(-1), rec["t31"]]).astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -304,7 +333,13 @@ def main():
     ap.add_argument("--strong-hyp", type=int, default=10000, help="strong-scaling leg: ONE round of this many hypotheses split over the GPUs (0 = skip)")
     ap.add_argument("--strong-hyp-large", type=int, default=100000, help="second strong-scaling point (0 = skip)")
     ap.add_argument("--no-host-class", action="store_true", help="skip the C++ GPU_HC_Solver leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of --impl ours computed to DIR/<name>.npy "
+                                                          "(at most 64 MB in all); not available with --impl reference")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return reference_arm(args)
 
@@ -417,6 +452,9 @@ def main():
     n_pred, n_corr = float(stats[:, 1].sum()), float(stats[:, 2].sum())
     flops_launch = FLOPS_PRED_STAGE * n_pred + FLOPS_CORR_STAGE * n_corr
     counts = hc.count_solutions(tracks, conv, inf, H)
+    if args.dump_outputs:
+        support = None if args.abort else trk.d_support[:n_paths].cpu().numpy()
+        dump_outputs(args.dump_outputs, rank, world, tracks, conv, inf, stats, support, round_record)
 
     # ---- the gather itself: NCCL all_gather of the 128-byte records vs D2H + host (gloo) exchange -------------------
     gather_cmp = None

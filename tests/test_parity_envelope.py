@@ -10,7 +10,8 @@ statistical gate, this module makes a PER-PATH statement:
   stochastic-arithmetic seeds (every linear-solve result moved by -1/0/+1 ulp).  A path whose flags differ between any two variants
   is UNSTABLE; the set is committed under tests/golden/envelope_*.npz.  It is computed WITHOUT looking at any reference result.
 * The tests then require that the paths on which this library (== the oracle spec, bit for bit: tests/test_gpu_full.py) differs from
-  - the reference GPU-HC++ kernels run live on the same GPU (pruning on, 100 and 1000 hypotheses; early abort),
+  - the reference GPU-HC++ kernels (pruning on, 100 and 1000 hypotheses: their flags from a B200 are committed under
+    tests/golden/ref_gpuhc_*.npz, and where oracle/_ref is built the kernels also run live and must reproduce them; early abort),
   - the unmodified reference CPU-HC (pruning off; committed golden of the real thing),
   - the reference CPU-HC with the GPU kernels' pruning patched in (pruning on; committed golden),
   lie in the unstable set, and that STABLE paths agree.  Flag flips have a long tail of rarely-flipping paths, so a finite number of
@@ -143,25 +144,43 @@ MIN_STABLE = {"gpu_h100": 0.9998, "gpu_h1000": 0.9999}
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# GPU tests: the reference GPU-HC++ kernels live, on the same GPU and inputs
+# GPU tests: this library live against the reference GPU-HC++ kernels on the same inputs
 
-def _run_both(problem, ransac0, H):
-    from oracle.pyoracle import ReferenceGPU, REF_GPU_SO
+def _round(problem, ransac0, H):
     from trifocal_pose_estimation_using_improved_gpuhc_b200 import hc
-    if not os.path.exists(REF_GPU_SO):
-        pytest.skip("oracle/_ref/libref_gpuhc.so not built")
     picked = hc.sample_hypotheses(0, H, ransac0["locations"].shape[0])
     target, diff = hc.target_params_from_picks(picked, ransac0["locations"], ransac0["tangents"], problem["start_params"])
-    ref = ReferenceGPU(problem)
-    ref.setup(target, diff, ransac0["locations"], ransac0["K"])
-    ref.track()
-    tr_r, cv_r, inf_r = ref.results()
+    return picked, target, diff
+
+
+def _run_ours(problem, ransac0, target, diff, H):
+    from trifocal_pose_estimation_using_improved_gpuhc_b200 import hc
     trk = hc.Tracker(problem=problem, stats=True)
     trk.set_edgels(ransac0["locations"], ransac0["K"])
     trk.upload_params(target, diff)
     trk.track(H, prune=True)
-    tr, cv, inf, st = trk.results(H)
-    return picked, (tr, cv, inf, st), (tr_r, cv_r, inf_r), trk, ref
+    return trk.results(H), trk
+
+
+def _run_reference_live(problem, ransac0, target, diff):
+    """The reference GPU-HC++ kernels themselves (oracle/_ref/libref_gpuhc.so, built only where the reference sources are present)."""
+    from oracle.pyoracle import ReferenceGPU
+    ref = ReferenceGPU(problem)
+    ref.setup(target, diff, ransac0["locations"], ransac0["K"])
+    ref.track()
+    return ref.results(), ref
+
+
+def _reference_flags(H):
+    """(converged, infinity, real) of the reference GPU-HC++ kernels on the seed-0 round, as committed from a B200 run."""
+    r = np.load(os.path.join(GOLD, "ref_gpuhc_seed0_h%d.npz" % H))
+    P = H * 312
+    return r["picked"], _bits(r["converged_bits"], P), _bits(r["infinity_bits"], P), _bits(r["real_bits"], P)
+
+
+def _ref_gpu_built():
+    from oracle.pyoracle import REF_GPU_SO
+    return os.path.exists(REF_GPU_SO)
 
 
 def _real(tr, cv):
@@ -171,19 +190,26 @@ def _real(tr, cv):
 @pytest.mark.gpu
 @pytest.mark.parametrize("H,key", [(100, "gpu_h100"), (1000, "gpu_h1000")])
 def test_differences_from_the_reference_gpu_kernels_are_unstable_paths(problem, ransac0, H, key):
+    """This library run live against the reference kernels' committed flags; where oracle/_ref is built, the reference kernels run
+    live too and must reproduce those flags (they are deterministic on one GPU)."""
     e = _load_env("envelope_seed0_h%d_prune.npz" % H)
     P = H * 312
-    picked, (tr, cv, inf, st), (tr_r, cv_r, inf_r), trk, ref = _run_both(problem, ransac0, H)
-    assert np.array_equal(picked, e["picked"])
+    picked, target, diff = _round(problem, ransac0, H)
+    (tr, cv, inf, st), trk = _run_ours(problem, ransac0, target, diff, H)
+    picked_r, cv_r, inf_r, real_r = _reference_flags(H)
+    assert np.array_equal(picked, e["picked"]) and np.array_equal(picked, picked_r)
+    if _ref_gpu_built():
+        (tr_l, cv_l, inf_l), _ = _run_reference_live(problem, ransac0, target, diff)
+        assert np.array_equal(cv_l != 0, cv_r) and np.array_equal(inf_l != 0, inf_r) and np.array_equal(_real(tr_l, cv_l), real_r)
     # this library IS the spec column of the envelope (bit-exact oracle parity, here re-checked on the flags)
     assert np.array_equal(np.packbits(cv), e["spec_conv"]) and np.array_equal(np.packbits(inf), e["spec_inf"])
     unstable = _bits(e["unstable"], P)
-    diff = (cv != cv_r) | (inf != inf_r) | (_real(tr, cv) != _real(tr_r, cv_r))
+    diff = ((cv != 0) != cv_r) | ((inf != 0) != inf_r) | (_real(tr, cv) != real_r)
     _check(diff, unstable, "reference GPU-HC++ kernels, %d hypotheses" % H, max_outside=MAX_OUTSIDE[key],
            min_coverage=MIN_COVERAGE[key], min_stable_agreement=MIN_STABLE[key])
     # per hypothesis: counts over the STABLE paths are identical in every hypothesis but the stragglers'
     s = ~unstable
-    for flag_a, flag_b in ((cv, cv_r), (inf, inf_r), (_real(tr, cv), _real(tr_r, cv_r))):
+    for flag_a, flag_b in ((cv, cv_r), (inf, inf_r), (_real(tr, cv), real_r)):
         a = (flag_a.astype(bool) & s).reshape(H, 312).sum(1)
         b = (flag_b.astype(bool) & s).reshape(H, 312).sum(1)
         assert (a != b).sum() <= MAX_OUTSIDE[key]
@@ -191,10 +217,12 @@ def test_differences_from_the_reference_gpu_kernels_are_unstable_paths(problem, 
 
 @pytest.mark.gpu
 def test_early_abort_results_are_the_no_abort_results_of_the_paths_that_ran(problem, ransac0):
-    """Abort mode adds no new kind of difference: a path that ran to completion before the flag went up has exactly its no-abort result
-    (ours: bit for bit; reference: its own no-abort flags), so per-path parity in abort mode is inherited from the no-abort round."""
+    """Abort mode adds no new kind of difference: a path that ran to completion before the flag went up has exactly its no-abort result,
+    bit for bit, so per-path parity in abort mode is inherited from the no-abort round.  The reference's side of this statement is
+    test_reference_early_abort_results_are_its_no_abort_results."""
     H = 100
-    picked, (tr, cv, inf, st), (tr_r, cv_r, inf_r), trk, ref = _run_both(problem, ransac0, H)
+    picked, target, diff = _round(problem, ransac0, H)
+    (tr, cv, inf, st), trk = _run_ours(problem, ransac0, target, diff, H)
     trk.track_abort(H, prune=True)
     tr_a, cv_a, inf_a, st_a = trk.results(H)
     ran = (st_a[:, 3] >> 16) < 4                       # not skipped / cut by the flag
@@ -202,10 +230,21 @@ def test_early_abort_results_are_the_no_abort_results_of_the_paths_that_ran(prob
     assert np.array_equal(cv_a[ran], cv[ran]) and np.array_equal(inf_a[ran], inf[ran])
     a, b = np.ascontiguousarray(tr_a[ran][:, :30]), np.ascontiguousarray(tr[ran][:, :30])
     assert bool(np.all((a.view(np.uint64) == b.view(np.uint64)) | (np.isnan(a) & np.isnan(b))))
+    best = trk.d_best.cpu().numpy()
+    assert best[0] == 1 and best[1] == 104             # stops on hypothesis 0 / track 104, the ground-truth pose
+
+
+@pytest.mark.gpu
+@pytest.mark.skipif(not _ref_gpu_built(), reason="oracle/_ref/libref_gpuhc.so not built (needs the reference sources at build time)")
+def test_reference_early_abort_results_are_its_no_abort_results(problem, ransac0):
+    """The reference kernels in abort mode: every path they report converged also converged without abort, and they stop on the same
+    ground-truth path as this library."""
+    H = 100
+    picked, target, diff = _round(problem, ransac0, H)
+    (_, cv_r, _), ref = _run_reference_live(problem, ransac0, target, diff)
     ref.reload()
     ref.track_abort()
     _, cv_ra, _ = ref.results()
     assert np.all(cv_r[cv_ra != 0] != 0)               # every path the reference reports converged under abort converged without it
     idx = ref.d_found_index.cpu().numpy()
-    best = trk.d_best.cpu().numpy()
-    assert best[0] == 1 and best[1] == 104 and 104 in idx[idx >= 0]      # both stop on hypothesis 0 / track 104, the ground-truth pose
+    assert 104 in idx[idx >= 0]
