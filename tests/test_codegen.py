@@ -143,32 +143,3 @@ def test_column_classes_partition_the_nonzero_columns():
     for cl in g["classes"]:
         for lane in range(30):
             assert sum((lane, c) in g["hx_terms"] for c in cl) <= 1
-
-
-def test_two_path_header_is_current_and_covers_every_term(tmp_path):
-    """The two-paths-per-warp layout (csrc/hc_problem_gen_tp.h, kernel variant -DHC_TWO_PATHS=1): the committed header is what the
-    generator emits, every row sits in exactly one (lane, row slot), and the per-row-slot schedules hold every non-zero term of
-    every row exactly once, in table order (so sums stay bit-identical to the oracle's)."""
-    g = gen_eval.build()
-    t = gen_eval.build_tp(g)
-    text = gen_eval.emit_tp(g, t, str(tmp_path / "tp.h"))
-    assert text == open(os.path.join(PKG, "csrc", "hc_problem_gen_tp.h")).read()
-    rows = [r for pair in t["row_at"] for r in pair if r >= 0]
-    assert sorted(rows) == list(range(30))
-    lane32 = g["lane_of_row"]
-    for ci in range(len(g["classes"])):
-        ref_rows = [row for (cc, row) in g["hx_slots"] if cc == ci]
-        for r in (0, 1):
-            mine = [rowp for (cc, rr, rowp) in t["hx_tp"] if cc == ci and rr == r]
-            for l in range(16):
-                row = t["row_at"][l][r]
-                got = [p[l] for p in mine if p[l] is not None]
-                want = [p[lane32[row]] for p in ref_rows if p[lane32[row]] is not None] if row >= 0 else []
-                assert got == want, (ci, r, l)
-    for r in (0, 1):
-        for l in range(16):
-            row = t["row_at"][l][r]
-            for mine, ref in ((t["h_tp"][r], g["h_slots"]), (t["ht_tp"][r], g["ht_slots"])):
-                got = [p[l] for p in mine if p[l] is not None]
-                want = [p[lane32[row]] for p in ref if p[lane32[row]] is not None] if row >= 0 else []
-                assert got == want, (r, l)

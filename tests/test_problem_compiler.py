@@ -99,13 +99,23 @@ def test_committed_header_is_what_the_compiler_emits(name, tmp_path):
         assert "#define HCG_K1 2 " in text                                           # block structure found in a non-trifocal system
 
 
-def test_trifocal_header_is_still_byte_identical_after_generalisation(tmp_path):
+def _csrc_snapshot():
+    csrc = os.path.join(PKG, "csrc")
+    snap = {}
+    for d, _, files in os.walk(csrc):
+        for f in files:
+            p = os.path.join(d, f)
+            with open(p, "rb") as fh:
+                snap[os.path.relpath(p, csrc)] = fh.read()
+    return snap
+
+
+def test_trifocal_header_is_byte_identical_and_the_generator_leaves_csrc_untouched(tmp_path):
     out = str(tmp_path / "gen.h")
-    tp = os.path.join(PKG, "csrc", "hc_problem_gen_tp.h")          # (the generator rewrites the two-paths header in place)
-    tp_before = open(tp).read()
+    before = _csrc_snapshot()                                      # the generator writes --out and nothing else: committed sources stay as they are
     subprocess.check_call([sys.executable, os.path.join(PKG, "codegen", "gen_eval.py"), "--out", out], stdout=subprocess.DEVNULL)
     assert open(out).read() == open(os.path.join(PKG, "csrc", "hc_problem_gen.h")).read()
-    assert open(tp).read() == tp_before
+    assert _csrc_snapshot() == before
 
 
 @pytest.mark.parametrize("name", PROBLEMS)

@@ -160,29 +160,7 @@ def level_schedule(hx_terms, K1, segments, seg_cols):
         shared = [c for c in range(K1, N) if need[c]]
         levels.append(here)
         first_shared.append(min(shared) if shared else N)
-    level_schedule.group_patterns = [(l, g, c, part, u) for (l, g, c, part, u) in groups]      # kept for store_limits()
     return levels, level_of_col, first_shared
-
-
-def store_limits(K1, nsp, nslot, lane_of_row):
-    """Per super-step T and slot pair (t, t+1): one past the highest lane whose pivot group can hold a non-zero in that pair (sparse slots and
-    the right-hand side pair count as always needed).  A pivot lane at or above the limit need not store the pair — its group's buffer keeps
-    the zeros it was initialised with — which matters because a 128-bit store costs one shared-memory wavefront per quarter-warp that holds a
-    storing lane."""
-    lim = [[32] * (nslot // 2) for _ in range(nsp)]
-    for T in range(nsp):
-        for pr in range(nslot // 2):
-            t = 2 * pr
-            if t < nsp:
-                continue                                  # pairs that hold sparse slots: keep unconditional
-            top = 0
-            for (l, g, c, part, u) in level_schedule.group_patterns:
-                if l != T:
-                    continue
-                if u[K1 + (t - nsp)] or u[K1 + (t + 1 - nsp)]:
-                    top = max(top, 1 + max(lane_of_row[r] for r in part))
-            lim[T][pr] = top if top > 0 else 32           # (untouched pairs are not stored at all: the limit is irrelevant)
-    return lim
 
 
 def column_classes(hx_terms):
@@ -366,7 +344,6 @@ def build():
     lane_of_row = [row_of_lane.index(r) for r in range(N)]
     nsp = len(levels)
     nd = N - K1
-    sp_store_limit = store_limits(K1, nsp, nsp + nd, lane_of_row) if nsp else []
     # per lane and level: the private column the lane's row meets there (or None), the lanes of its group (6-bit mask relative
     # to the segment's first lane) and the group's index within the segment (selects the pivot-row buffer)
     col_at = [[None] * nsp for _ in range(WARP)]
@@ -518,7 +495,7 @@ def build():
     return dict(hx_terms=hx_terms, h_terms=h_terms, cq_list=cq_list, dq_list=dq_list, classes=classes,
                 col_class=col_class, hx_slots=hx_slots, h_slots=h_slots, ht_slots=ht_slots,
                 K1=K1, segments=segments, seg_cols=seg_cols, row_of_lane=row_of_lane, lane_of_row=lane_of_row,
-                nsp=nsp, nd=nd, nslot=nslot, sp_first_shared=sp_first_shared, sp_store_limit=sp_store_limit, levels=levels, level_of_col=level_of_col,
+                nsp=nsp, nd=nd, nslot=nslot, sp_first_shared=sp_first_shared, levels=levels, level_of_col=level_of_col,
                 col_at=col_at, grp_mask=grp_mask, grp_sub=grp_sub, max_sub=max_sub, scatter=scatter, sel_of_lane=sel_of_lane, nz_of_lane=nz_of_lane, n_sel=n_sel,
                 pairs=pair_by_pos, triples=tri_by_pos, XP_PAIR0=XP_PAIR0, XP_TRI0=XP_TRI0, XP_TOTAL=XP_TOTAL,
                 layout_cost=layout_cost)
@@ -662,247 +639,11 @@ def emit(g, path):
     for t, (ca, cb, sb) in enumerate(g["scatter"]):
         w("  X(%d, %d, %d, %d) \\" % (t, ca, cb, sb))
     w("")
-    w("// per super-step and slot pair: pivot lanes at or above this lane never hold a non-zero there and skip the store (32: everybody stores)")
-    w("#define HCG_SP_STORE_LIMIT_INIT { " + ", ".join("{" + ",".join(str(v) for v in row) + "}" for row in (g["sp_store_limit"] or [[32] * (g["nslot"] // 2)])) + " }")
     w("// problem identity: the kernel takes every size from this header (codegen/gen_eval.py --problem-dir compiles another problem)")
     w("#define HCG_PROBLEM_NAME \"%s\"" % SPEC["name"])
     w("#define HCG_TRACKS %d        /* homotopy paths per hypothesis (Num_Of_Tracks) */" % SPEC["n_tracks"])
     w("#define HCG_NUM_DEPTHS %d      /* leading variables that are depths: positive-depth pruning tests them (0: no pruning) */" % SPEC["n_depths"])
     w("#define HCG_TRIFOCAL %d        /* 1: the trifocal relative-pose problem (in-kernel scoring, pose records, target-parameter gather) */" % SPEC["trifocal"])
-    w("")
-    w("#endif")
-    text = "\n".join(L) + "\n"
-    with open(path, "w") as f:
-        f.write(text)
-    return text
-
-
-# =====================================================================================================================
-# Two paths per warp, two rows per lane ("TP" layout, csrc/hc_tracker.cu hc_track_tp_kernel).
-# A half-warp (16 lanes) tracks one path; lane l of the half holds TWO matrix rows (row slots 0 and 1) and the two variables l and
-# l + 16.  A 6-row segment of the block structure sits on three consecutive lanes: rows seg[0..2] in slot 0, seg[3..5] in slot 1;
-# lane 15 is idle.  The pivot row of an elimination step is then loaded once per lane and applied to two rows, and one warp
-# instruction serves two paths — about a quarter fewer shared-memory wavefronts and an eighth fewer instructions per path.
-# Everything a row computes (term order, pivot rule, update arithmetic) is unchanged, so results stay bit-identical to the oracle.
-HALF = 16
-SEG_LANES = 3
-
-
-def build_tp(g):
-    segs = g["segments"]
-    assert len(segs) * SEG_LANES <= HALF and all(len(sg) == 6 for sg in segs)
-    row_at = [[-1, -1] for _ in range(HALF)]            # row_at[lane][slot]
-    for gi, sg in enumerate(segs):
-        for i in range(SEG_LANES):
-            row_at[gi * SEG_LANES + i][0] = sg[i]
-            row_at[gi * SEG_LANES + i][1] = sg[i + SEG_LANES]
-    pos_of_row = {row_at[l][r]: (l, r) for l in range(HALF) for r in (0, 1) if row_at[l][r] >= 0}
-    nsp, K1 = g["nsp"], g["K1"]
-    # per level: pivot groups.  Every group must be exactly the slot-0 rows of a segment, its slot-1 rows, or all six ("merged").
-    lvl = [[dict(a0=0, a1=0, merged=0, buf0=0, buf1=0, col0=None, col1=None) for _ in range(nsp)] for _ in range(HALF)]
-    n_buf = [0] * nsp
-    for T, here in enumerate(g["levels"]):
-        nb = 0
-        for (gi, c, part) in here:
-            lanes = range(gi * SEG_LANES, gi * SEG_LANES + SEG_LANES)
-            s0 = [row_at[l][0] for l in lanes]
-            s1 = [row_at[l][1] for l in lanes]
-            part = sorted(part)
-            if part == sorted(s0 + s1):
-                for l in lanes:
-                    lvl[l][T].update(a0=1, a1=1, merged=1, buf0=nb, buf1=nb, col0=c, col1=c)
-            elif part == sorted(s0):
-                for l in lanes:
-                    lvl[l][T].update(a0=1, buf0=nb, col0=c)
-            elif part == sorted(s1):
-                for l in lanes:
-                    lvl[l][T].update(a1=1, buf1=nb, col1=c)
-            else:
-                raise AssertionError("pivot group %s of level %d does not map onto row slots" % (part, T))
-            nb += 1
-        n_buf[T] = nb
-    max_buf = max(n_buf)
-
-    def slot_of(row, col):
-        if col >= K1:
-            return nsp + (col - K1)
-        return g["level_of_col"][col]
-
-    # ---- evaluator schedules per row slot (16 lanes each) ----------------------------------------------------------
-    classes, col_class, hx_terms, h_terms = g["classes"], g["col_class"], g["hx_terms"], g["h_terms"]
-    # the 32-lane build already fixed table POSITIONS (bank-conflict search): reuse its packed payloads through the lane of the row
-    lane32_of_row = g["lane_of_row"]
-    hx_by_class = {}
-    for ci in range(len(classes)):
-        hx_by_class[ci] = [row for (cc, row) in g["hx_slots"] if cc == ci]         # rows of 32 payloads, in slot order
-
-    def row_seq(slot_rows, row):
-        """the payload sequence of one matrix row out of the 32-lane slot rows"""
-        ln = lane32_of_row[row]
-        return [r[ln] for r in slot_rows if r[ln] is not None]
-
-    hx_tp = []      # (class, slot r, [16 payloads])
-    for ci in range(len(classes)):
-        for r in (0, 1):
-            seqs = [row_seq(hx_by_class[ci], row_at[l][r]) if row_at[l][r] >= 0 else [] for l in range(HALF)]
-            for rowp in schedule(seqs) if any(seqs) else []:
-                hx_tp.append((ci, r, rowp))
-    h_tp, ht_tp = [], []
-    for r in (0, 1):
-        seqs = [row_seq(g["h_slots"], row_at[l][r]) if row_at[l][r] >= 0 else [] for l in range(HALF)]
-        h_tp.append(schedule(seqs))
-        seqs = [row_seq(g["ht_slots"], row_at[l][r]) if row_at[l][r] >= 0 else [] for l in range(HALF)]
-        ht_tp.append(schedule(seqs))
-    assert len(h_tp[0]) == len(h_tp[1]) == len(ht_tp[0]) == len(ht_tp[1]), "H / Ht share one slot loop per row slot"
-
-    # ---- scatter of class accumulators into register slots, per row slot ------------------------------------------------
-    nslot = g["nslot"]
-    scatter, sel, nz = [], [[0, 0] for _ in range(HALF)], [[0, 0] for _ in range(HALF)]
-    n_sel = 0
-    for t in range(nslot):
-        cls = {}
-        for l in range(HALF):
-            for r in (0, 1):
-                row = row_at[l][r]
-                if row < 0:
-                    continue
-                if t < nsp:
-                    col = lvl[l][t]["col%d" % r]
-                else:
-                    col = K1 + (t - nsp)
-                if col is not None:
-                    cls[(l, r)] = col_class.get(col)
-        used = sorted({c for c in cls.values() if c is not None})
-        assert 1 <= len(used) <= 2
-        if len(used) == 1:
-            scatter.append((used[0], -1, -1))
-        else:
-            scatter.append((used[0], used[1], n_sel))
-            for (l, r), c in cls.items():
-                if c == used[1]:
-                    sel[l][r] |= 1 << n_sel
-            n_sel += 1
-    for l in range(HALF):
-        for r in (0, 1):
-            row = row_at[l][r]
-            if row < 0:
-                continue
-            for c in range(N):
-                if (row, c) in hx_terms:
-                    nz[l][r] |= 1 << slot_of(row, c)
-    return dict(row_at=row_at, lvl=lvl, n_buf=n_buf, max_buf=max_buf, hx_tp=hx_tp, h_tp=h_tp, ht_tp=ht_tp, scatter=scatter, sel=sel, nz=nz,
-                n_sel=n_sel)
-
-
-def emit_tp(g, t, path):
-    ncq, ndq = len(g["cq_list"]), len(g["dq_list"])
-    rounds = lambda n: (n + HALF - 1) // HALF
-    L = []
-    w = L.append
-    w("// GENERATED by codegen/gen_eval.py (two-paths-per-warp layout) — do not edit.  Companion of hc_problem_gen.h: same tables,")
-    w("// same table positions, re-scheduled for 16 lanes x 2 row slots per path.")
-    w("#ifndef HC_PROBLEM_GEN_TP_H")
-    w("#define HC_PROBLEM_GEN_TP_H")
-    nsp, nslot = g["nsp"], g["nslot"]
-    pairs, triples = g["pairs"], g["triples"]
-    rows = []
-
-    def add(words16):
-        """one table row = 16 words (one per lane of a half-warp); returns its index"""
-        assert len(words16) == HALF
-        rows.append(list(words16))
-        return len(rows) - 1
-
-    off_cq = len(rows)
-    for r in range(rounds(ncq)):
-        add([pack_build_word(g["cq_list"][r * HALF + l]) if r * HALF + l < ncq else pack_build_word((0, P_PAD, P_PAD)) for l in range(HALF)])
-    off_dq = len(rows)
-    for r in range(rounds(ndq)):
-        add([pack_build_word(g["dq_list"][r * HALF + l]) if r * HALF + l < ndq else pack_build_word((0, P_PAD, P_PAD)) for l in range(HALF)])
-    off_pair = len(rows)
-    for r in range(rounds(len(pairs))):
-        add([pack_xp_word(pairs[r * HALF + l]) if r * HALF + l < len(pairs) and pairs[r * HALF + l] is not None else pack_xp_word([]) for l in range(HALF)])
-    off_tri = len(rows)
-    for r in range(rounds(len(triples))):
-        add([pack_xp_word(triples[r * HALF + l]) if r * HALF + l < len(triples) and triples[r * HALF + l] is not None else pack_xp_word([]) for l in range(HALF)])
-    # Hx: for every (class, row slot) a contiguous run of table rows
-    hx_beg = {}
-    for ci in range(len(g["classes"])):
-        for r in (0, 1):
-            hx_beg[(ci, r)] = len(rows)
-            for (cc, rr, rowp) in t["hx_tp"]:
-                if cc == ci and rr == r:
-                    add([pack_word(p) for p in rowp])
-    hx_end = len(rows)
-    off_h, off_ht = [0, 0], [0, 0]
-    for r in (0, 1):
-        off_h[r] = len(rows)
-        for rowp in t["h_tp"][r]:
-            add([pack_word(p) for p in rowp])
-    for r in (0, 1):
-        off_ht[r] = len(rows)
-        for rowp in t["ht_tp"][r]:
-            add([pack_word(p) for p in rowp])
-    w("#define HCT_CQ_ROUNDS %d" % rounds(ncq))
-    w("#define HCT_DQ_ROUNDS %d" % rounds(ndq))
-    w("#define HCT_PAIR_ROUNDS %d" % rounds(len(pairs)))
-    w("#define HCT_TRI_ROUNDS %d" % rounds(len(triples)))
-    w("#define HCT_TBL_CQ %d" % off_cq)
-    w("#define HCT_TBL_DQ %d" % off_dq)
-    w("#define HCT_TBL_PAIR %d" % off_pair)
-    w("#define HCT_TBL_TRI %d" % off_tri)
-    w("#define HCT_RHS_SLOTS %d   /* H and Ht term slots per row slot */" % len(t["h_tp"][0]))
-    w("#define HCT_TBL_H_INIT { %d, %d }    /* first table row of H for row slot 0 / 1 */" % tuple(off_h))
-    w("#define HCT_TBL_HT_INIT { %d, %d }" % tuple(off_ht))
-    # class begin table: [class][slot] -> first row, and the end
-    begs = []
-    for ci in range(len(g["classes"])):
-        for r in (0, 1):
-            begs.append(hx_beg[(ci, r)])
-    begs.append(hx_end)
-    w("#define HCT_HX_BEGIN_INIT { " + ",".join(str(b) for b in begs) + " }   /* first table row of (class, row slot) = [2*class + slot], then the end */")
-    w("#define HCT_TBL_ROWS %d   /* rows of 16 words */" % len(rows))
-    w("#define HCT_TBL_INIT { \\")
-    for r in rows:
-        w("  " + ",".join("0x%08xu" % v for v in r) + ", \\")
-    w("}")
-    w("// lane l of a half-warp holds rows ROW_AT[l][0] and ROW_AT[l][1] (-1: none) and the variables l and l + 16")
-    w("#define HCT_ROW_AT_INIT { " + ",".join("%d,%d" % tuple(x) for x in t["row_at"]) + " }")
-    # per lane, per row slot: nz mask over register slots | selector bits << 20
-    w("#define HCT_LANEINFO_INIT { " + ",".join("0x%08xu,0x%08xu" % (t["nz"][l][0] | (t["sel"][l][0] << 20), t["nz"][l][1] | (t["sel"][l][1] << 20)) for l in range(HALF)) + " }")
-    # per lane, per row slot: the private column met on every level, 5 bits each
-    cols = []
-    for l in range(HALF):
-        for r in (0, 1):
-            v = 0
-            for T in range(nsp):
-                c = t["lvl"][l][T]["col%d" % r]
-                if c is not None:
-                    v |= c << (5 * T)
-            cols.append(v)
-    w("#define HCT_LANECOLS_INIT { " + ",".join("0x%08xu" % v for v in cols) + " }")
-    # per lane, per level (8 bits): active0 | active1 << 1 | merged << 2 | buf0 << 3 | buf1 << 5 ... buffers < 8: 3 bits each -> 9 bits; use 16 bits per level
-    assert t["max_buf"] <= 8 and nsp <= 4
-    lv = []
-    for l in range(HALF):
-        lo = 0
-        for T in range(nsp):
-            d = t["lvl"][l][T]
-            word = d["a0"] | (d["a1"] << 1) | (d["merged"] << 2) | (d["buf0"] << 3) | (d["buf1"] << 6)
-            lo |= word << (16 * (T % 2)) if False else 0
-        # two 32-bit words: levels 0,1 in the first, 2,3 in the second
-        ws = [0, 0]
-        for T in range(nsp):
-            d = t["lvl"][l][T]
-            word = d["a0"] | (d["a1"] << 1) | (d["merged"] << 2) | (d["buf0"] << 3) | (d["buf1"] << 6)
-            ws[T // 2] |= word << (16 * (T % 2))
-        lv.append(ws)
-    w("#define HCT_LANELVL_INIT { " + ",".join("0x%08xu,0x%08xu" % tuple(x) for x in lv) + " }   /* 16 bits per level: active0 | active1<<1 | merged<<2 | buf0<<3 | buf1<<6 */")
-    w("#define HCT_MAX_BUF %d   /* pivot-row buffers per parity */" % t["max_buf"])
-    w("// X(slot, classA, classB, selbit): A[slot] = row has a non-zero there ? acc[selbit set ? classB : classA] : 0")
-    w("#define HCT_HX_SCATTER_LIST(X) \\")
-    for tt, (ca, cb, sb) in enumerate(t["scatter"]):
-        w("  X(%d, %d, %d, %d) \\" % (tt, ca, cb, sb))
     w("")
     w("#endif")
     text = "\n".join(L) + "\n"
@@ -940,11 +681,6 @@ def main():
     g = build()
     out = a.out or os.path.join(PKG, "csrc", "hc_problem_gen.h")
     emit(g, out)
-    t = build_tp(g)
-    emit_tp(g, t, os.path.join(PKG, "csrc", "hc_problem_gen_tp.h"))
-    print("two-path layout: row_at", t["row_at"], "buffers per level", t["n_buf"], "Hx table rows per (class, slot)",
-          [(ci, r, sum(1 for (cc, rr, _) in t["hx_tp"] if cc == ci and rr == r)) for ci in range(len(g["classes"])) for r in (0, 1)],
-          "rhs slots", len(t["h_tp"][0]), "scatter", t["scatter"])
     print("classes:", g["classes"])
     print("K1 %d segments %s seg_cols %s" % (g["K1"], g["segments"], g["seg_cols"]))
     print("row_of_lane", g["row_of_lane"])
