@@ -131,6 +131,42 @@ int hcb200_track_abort_peers(void* stream, int n_hyp, int n_edgels,
                        hcb200_path_stats* d_stats, void* d_workspace,
                              uint8_t* const* d_peer_found, int n_peers);
 
+/* Early-abort rounds of MANY image triplets ("problems": dataset, edgel set, K) in one launch.  An abort round is bound by the latency of
+ * one long path (~80 HC steps) while most resident warps track hypotheses whose work the flag then throws away; here the queue interleaves
+ * the problems, so the first wave of warps holds the first hypotheses of every problem and K early-hit problems end in about the time of one.
+ * Every problem has n_hyp_per_problem hypotheses.
+ *   Storage is problem-major: path id b = problem * n_hyp_per_problem * 312 + hypothesis * 312 + track, so each problem's target / diff
+ *     parameters ([n_problems * n_hyp_per_problem][34]), tracks, flags, stats and found indices form one contiguous slice.  d_found_index
+ *     [all paths] is pre-set to -1 by the caller; entry b becomes b (the storage id) when path b passes.
+ *   The queue is interleaved: queue position q tracks problem q % n_problems, local path q / n_problems.  Within a problem, paths start in
+ *     the order of a single-problem launch.  The order is fixed.
+ *   Each problem has its own early abort: d_found [n_problems] uint8, 0 on entry.  A passing path of problem k raises only d_found[k]; the
+ *     paths of problem k poll only that byte, at path start and at every HC step, like hcb200_track_abort.  Skipped paths of a problem are
+ *     as there: converged = 0, infinity = 0, end reason 4.  The pass test is hcb200_track_abort's, against problem k's edgels
+ *     [off[k], off[k+1]) of d_edgel_locations ([off[n_problems]][6]) and its K, d_intrinsics + 9 k ([n_problems][9] row-major).
+ *   Each problem has its own result: d_best [n_problems] (may be NULL) receives problem k's record: found, smallest passing path id LOCAL to
+ *     the problem (hypothesis * 312 + track), its inlier counts, n_passed.  The layout is hcb200_track_abort's, so
+ *     hcb200_make_pose_record(d_tracks + 62 * 312 * n_hyp_per_problem * k, d_best + k, d_found + k, path_offset, rank, ...) works on the slice.
+ *     An empty round (n_hyp_per_problem == 0) clears every record.
+ *   h_edgel_offsets is a HOST array [n_problems + 1]: off[0] == 0, problem k owns edgels [off[k], off[k+1]).  The launcher copies it into the
+ *     workspace (cudaMemcpyAsync from pageable memory: the array may be reused when the call returns).  d_workspace holds
+ *     hcb200_batch_workspace_bytes(n_problems) = 256 + 16 * (n_problems + 1) bytes: per-problem best keys, pass counters and edgel offsets.
+ *   flags: HCB200_FLAG_PRUNE_PATHS; the split flag is ignored, as in hcb200_track_abort.
+ * Returns cudaErrorInvalidValue, before any CUDA call and with nothing launched, for NULL buffers (d_best and d_stats may be NULL),
+ * n_problems outside [1, HCB200_BATCH_MAX_PROBLEMS], n_hyp_per_problem < 0, n_problems * n_hyp_per_problem > 3 441 480 (31-bit path ids),
+ * hc_max_correction_steps < 1, off[0] != 0, or a problem with 0 or more than 65 535 edgels.  cudaErrorNotSupported in a compiled-problem
+ * library.  The limit on n_problems keeps the staged offsets (16 bytes per problem) in one 64 KB copy. */
+#define HCB200_BATCH_MAX_PROBLEMS 4095
+size_t hcb200_batch_workspace_bytes(int n_problems);
+int hcb200_track_abort_batched(void* stream, int n_problems, int n_hyp_per_problem, const int32_t* h_edgel_offsets,
+                               int hc_max_steps, int hc_max_correction_steps, int hc_delta_t_incremental_steps, unsigned flags,
+                               const float* d_start_sols, const float* d_start_params,
+                               const float* d_target_params, const float* d_diff_params,
+                               const float* d_edgel_locations, const float* d_intrinsics,
+                               float* d_tracks, uint8_t* d_converged, uint8_t* d_infinity,
+                               uint8_t* d_found, int32_t* d_found_index, hcb200_best_record* d_best,
+                               hcb200_path_stats* d_stats, void* d_workspace);
+
 /* Lets kernels running on `device` store into memory of `peer_device` (cudaDeviceEnablePeerAccess in `device`'s context; "already enabled" is
  * success; cudaErrorPeerAccessUnsupported when the two GPUs have no peer path).  Needed once per ordered pair before hcb200_track_abort_peers. */
 int hcb200_enable_peer_access(int device, int peer_device);

@@ -27,7 +27,9 @@ _lib = None
 ABI_SYMBOLS = ("hcb200_workspace_bytes", "hcb200_abi_version", "hcb200_track", "hcb200_track_abort",
                "hcb200_build_target_params", "hcb200_score_tracks", "hcb200_refine_tracks", "hcb200_kernel_info", "hcb200_ffma_probe",
                "hcb200_error_string", "hcb200_make_pose_record", "hcb200_reduce_pose_records", "hcb200_count_solutions", "hcb200_problem_info",
-               "hcb200_workspace_bytes_for", "hcb200_track_abort_peers", "hcb200_enable_peer_access")
+               "hcb200_workspace_bytes_for", "hcb200_track_abort_peers", "hcb200_enable_peer_access", "hcb200_batch_workspace_bytes",
+               "hcb200_track_abort_batched")
+BATCH_MAX_PROBLEMS = 4095      # HCB200_BATCH_MAX_PROBLEMS
 
 
 class HCB200Error(RuntimeError):
@@ -57,6 +59,10 @@ def load_library(path=None):
     lib.hcb200_track_abort.argtypes = [vp, i32, i32, i32, i32, i32, u32] + [vp] * 14
     lib.hcb200_track_abort_peers.restype = i32
     lib.hcb200_track_abort_peers.argtypes = [vp, i32, i32, i32, i32, i32, u32] + [vp] * 14 + [ctypes.POINTER(vp), i32]
+    lib.hcb200_batch_workspace_bytes.restype = ctypes.c_size_t
+    lib.hcb200_batch_workspace_bytes.argtypes = [i32]
+    lib.hcb200_track_abort_batched.restype = i32
+    lib.hcb200_track_abort_batched.argtypes = [vp, i32, i32, vp, i32, i32, i32, u32] + [vp] * 14
     lib.hcb200_enable_peer_access.restype = i32
     lib.hcb200_enable_peer_access.argtypes = [i32, i32]
     lib.hcb200_build_target_params.restype = i32
@@ -263,6 +269,78 @@ class Tracker:
                 rc = self.lib.hcb200_track_abort(*args)
         _check(rc, "hcb200_track_abort")
         self.launches += 2
+
+    # ---- early-abort rounds of many image triplets ("problems") in one launch (hcb200_track_abort_batched).  The parameters are uploaded
+    # stacked problem-major (upload_params of [n_problems * n_hyp, 34]); tracks, flags, stats and found indices come back in the same order.
+
+    def set_edgel_batch(self, locations_list, K_list):
+        """Problem k's edgel locations [E_k, 6] and 3x3 intrinsics: concatenated and uploaded; the host keeps the edgel offsets."""
+        torch = self.torch
+        locs = [np.ascontiguousarray(loc, np.float32).reshape(-1, 6) for loc in locations_list]
+        if len(locs) != len(K_list) or not locs:
+            raise ValueError("one K per edgel set, at least one problem")
+        self.batch_offsets = np.concatenate([[0], np.cumsum([loc.shape[0] for loc in locs])]).astype(np.int32)
+        self.d_edgels_batch = torch.from_numpy(np.concatenate(locs)).to(self.device)
+        self.d_K_batch = torch.from_numpy(np.stack([np.asarray(K, np.float32).reshape(9) for K in K_list])).to(self.device)
+
+    def _reserve_batch(self, n_problems):
+        torch = self.torch
+        if getattr(self, "d_found_batch", None) is not None and self.d_found_batch.shape[0] >= n_problems:
+            return
+        self.d_found_batch = torch.zeros(n_problems, dtype=torch.uint8, device=self.device)
+        self.d_best_batch = torch.zeros((n_problems, 16), dtype=torch.int32, device=self.device)
+        self.d_ws_batch = torch.zeros(int(self.lib.hcb200_batch_workspace_bytes(n_problems)), dtype=torch.uint8, device=self.device)
+
+    def reset_abort_batched(self, n_problems, n_hyp):
+        """Clear the problems' early-abort flags and the found indices of their paths."""
+        self._reserve_batch(n_problems)
+        self.d_found_batch[:n_problems].zero_()
+        self.d_found_index[:n_problems * n_hyp * NUM_TRACKS].fill_(-1)
+
+    def track_abort_batched(self, n_problems, n_hyp, prune=True):
+        """Early-abort rounds of the first n_problems problems of set_edgel_batch, n_hyp hypotheses each, in one launch; every problem stops on
+        its own first passing path.  Resets the flags and the found indices, then enqueues the launch; batch_records reads the results."""
+        if n_problems > len(self.batch_offsets) - 1:
+            raise ValueError("%d problems, but set_edgel_batch gave %d" % (n_problems, len(self.batch_offsets) - 1))
+        p = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
+        self.reset_abort_batched(n_problems, n_hyp)
+        offsets = np.ascontiguousarray(self.batch_offsets[:n_problems + 1])
+        with self.torch.cuda.device(self.device):
+            rc = self.lib.hcb200_track_abort_batched(
+                self._stream(), n_problems, n_hyp, offsets.ctypes.data_as(ctypes.c_void_p), self.max_steps, self.max_corr, self.dt_inc,
+                FLAG_PRUNE_PATHS if prune else 0, p(self.d_start_sols), p(self.d_start_params), p(self.d_target), p(self.d_diff),
+                p(self.d_edgels_batch), p(self.d_K_batch), p(self.d_tracks), p(self.d_conv), p(self.d_inf), p(self.d_found_batch),
+                p(self.d_found_index), p(self.d_best_batch), p(self.d_stats), p(self.d_ws_batch))
+        _check(rc, "hcb200_track_abort_batched")
+        self.launches += 2
+
+    def batch_records(self, n_problems):
+        """Synchronise and return the problems' best records: found, path_id (local to the problem: hypothesis * 312 + track, -1 when none),
+        inliers21, inliers31, n_passed."""
+        self.torch.cuda.synchronize(self.device)
+        best = self.d_best_batch[:n_problems].cpu().numpy()
+        return [dict(found=int(b[0]), path_id=int(b[1]), inliers21=int(b[2]), inliers31=int(b[3]), n_passed=int(b[4])) for b in best]
+
+    def score_tracks_batched(self, n_problems, n_hyp):
+        """No-abort counterpart of track_abort_batched: hcb200_score_tracks on each problem's slice of the last round, with the problem's edgels
+        and K.  Returns (support int32 [n_problems * n_hyp * 312, 2], best records int32 [n_problems, 16], path ids local to each problem)."""
+        torch = self.torch
+        L = n_hyp * NUM_TRACKS
+        if getattr(self, "d_support", None) is None or self.d_support.shape[0] < n_problems * L:
+            self.d_support = torch.empty((n_problems * L, 2), dtype=torch.int32, device=self.device)
+        self._reserve_batch(n_problems)
+        p = lambda t: ctypes.c_void_p(t.data_ptr())
+        off = self.batch_offsets
+        with torch.cuda.device(self.device):
+            for k in range(n_problems):
+                s = slice(k * L, (k + 1) * L)
+                rc = self.lib.hcb200_score_tracks(self._stream(), L, p(self.d_tracks[s]), p(self.d_conv[s]), int(off[k + 1] - off[k]),
+                                                  p(self.d_edgels_batch[int(off[k]):]), p(self.d_K_batch[k]), p(self.d_support[s]),
+                                                  p(self.d_best_batch[k]), p(self.d_ws))
+                _check(rc, "hcb200_score_tracks")
+                self.launches += 2
+        torch.cuda.synchronize(self.device)
+        return self.d_support[:n_problems * L].cpu().numpy(), self.d_best_batch[:n_problems].cpu().numpy()
 
     def refine_tracks(self, n_hyp, iters=3):
         """Device-side Newton refinement of the converged end points of the last round against their target systems (in place).
