@@ -13,7 +13,7 @@ LIBDIR := $(PKG)/lib
 CSRC   := $(PKG)/csrc
 HOST   := $(PKG)/host
 
-.PHONY: all product oracle ref clean
+.PHONY: all product oracle ref unit clean
 all: product
 product: $(LIBDIR)/libhcb200.so $(LIBDIR)/libhcb200_host.so $(LIBDIR)/hc-main
 
@@ -33,6 +33,18 @@ $(LIBDIR)/libhcb200_$(PROBLEM_NAME).so: $(CSRC)/hc_tracker.cu $(CSRC)/hc_problem
 	mkdir -p $(LIBDIR)
 	$(NVCC) $(NVFLAGS) -Xptxas -v -DHC_PROBLEM_HEADER='"hc_problem_gen_$(PROBLEM_NAME).h"' -shared -o $@ $(CSRC)/hc_tracker.cu \
 	  2> $(LIBDIR)/ptxas_hc_tracker_$(PROBLEM_NAME).log || (cat $(LIBDIR)/ptxas_hc_tracker_$(PROBLEM_NAME).log; false)
+
+# Test-only builds of the same source with the device primitives exposed (-DHC_UNIT; tests/test_device_primitives.py), with the product's
+# NVFLAGS: the trifocal problem (`make unit`) and any compiled problem (`make unit_problem PROBLEM_DIR=problems/<name>`).  Never shipped.
+unit: $(LIBDIR)/libhcb200_unit.so
+$(LIBDIR)/libhcb200_unit.so: $(CSRC)/hc_tracker.cu $(CSRC)/hc_problem_gen.h include/hcb200.h
+	mkdir -p $(LIBDIR)
+	$(NVCC) $(NVFLAGS) -DHC_UNIT -shared -o $@ $(CSRC)/hc_tracker.cu
+.PHONY: unit_problem
+unit_problem: $(LIBDIR)/libhcb200_unit_$(PROBLEM_NAME).so
+$(LIBDIR)/libhcb200_unit_$(PROBLEM_NAME).so: $(CSRC)/hc_tracker.cu $(CSRC)/hc_problem_gen_$(PROBLEM_NAME).h include/hcb200.h
+	mkdir -p $(LIBDIR)
+	$(NVCC) $(NVFLAGS) -DHC_UNIT -DHC_PROBLEM_HEADER='"hc_problem_gen_$(PROBLEM_NAME).h"' -shared -o $@ $(CSRC)/hc_tracker.cu
 
 HOST_SRCS := $(HOST)/GPU_HC_Solver.cpp $(HOST)/Data_Reader.cpp $(HOST)/Evaluations.cpp $(HOST)/host_capi.cpp
 HOST_HDRS := $(wildcard $(HOST)/*.hpp) include/hcb200.h

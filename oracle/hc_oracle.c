@@ -41,6 +41,7 @@ static inline hco_c32 c_recip(hco_c32 z)
   float q = 1.0f / d;
   return c_make(z.re * q, -(z.im * q));
 }
+void hco_recip(const hco_c32* z, hco_c32* out, int n) { for (int i = 0; i < n; i++) out[i] = c_recip(z[i]); }
 static inline uint32_t f_bits(float f) { uint32_t u; memcpy(&u, &f, 4); return u; }
 /* pivot key as the device sees it: NaN is the canonical 0x7fffffff */
 static inline uint32_t key_bits(float f) { return (f != f) ? 0x7fffffffu : f_bits(f); }

@@ -83,6 +83,7 @@ void hco_eval_H(const int* dHdt, const hco_c32* x31, const hco_c32* p34, hco_c32
 void hco_param_homotopy(float t, const hco_c32* start34, const hco_c32* target34, hco_c32* p34);
 
 /* linear solves: A row-major 30x30 (destroyed), b in / x out.  Return 0, or k+1 if the k-th pivot was exactly zero. */
+void hco_recip(const hco_c32* z, hco_c32* out, int n);   /* the spec's 1/z (conj(z) / clamp(|z|^2, 2^-100, 2^100)), element-wise */
 int hco_solve(hco_c32* A, hco_c32* b);          /* the spec: partial-pivot elimination, U-solve folded into the sweep */
 int hco_solve_lu_ref(hco_c32* A, hco_c32* b);   /* literal dev-cgesv-batched-small.cuh order (LU + back substitution) */
 
