@@ -49,7 +49,11 @@ extern "C" {
 #define HCB200_FLAG_SPLIT_LONG_PATHS 2u
 
 /* Optional per-path counters (all int32): HC steps attempted, predictor stages, corrector stages,
- * rejected steps | end reason << 16 (0 converged, 1 infinity, 2 pruned, 3 step cap, 4 skipped after abort). */
+ * rejected steps | end reason << 16 (0 converged, 1 infinity, 2 pruned, 3 step cap, 4 skipped after abort).
+ * The kernel counts in one packed word that holds at most 1 023 steps and 4 095 corrector stages per path.  A path takes up to
+ * hc_max_steps + 1 steps of up to hc_max_correction_steps corrector stages each, so every track entry point refuses a non-NULL
+ * d_stats (cudaErrorInvalidValue, nothing launched) when hc_max_steps > 1022 or (hc_max_steps + 1) * hc_max_correction_steps > 4095.
+ * Without stats these caps are free, except that hc_max_steps == INT_MAX and hc_max_correction_steps > INT_MAX - 4 are always refused. */
 typedef struct { int32_t steps, pred_stages, corr_stages, rejected_reason; } hcb200_path_stats;
 
 /* Best candidate of an early-abort launch, reduced on the device (64 bytes). */
@@ -88,7 +92,9 @@ int hcb200_problem_info(int* n_vars, int* n_params, int* n_tracks, int* is_trifo
 
 /* Replaces kernel_GPUHC_trifocal_2op1p_30x30_PH_CodeOpt_TrunPaths (…TrunPaths.cu:292-386).
  * Tracks all 312*n_hyp paths in one launch (0 <= n_hyp <= 3 441 480: path ids are 31-bit).  `stats` may be NULL.
- * Returns a cudaError_t value (0 == success; cudaErrorInvalidValue for NULL buffers or out-of-range counts, nothing launched). */
+ * Returns a cudaError_t value (0 == success; cudaErrorInvalidValue for NULL buffers or out-of-range counts, nothing launched).
+ * Out of range: n_hyp, hc_max_correction_steps < 1, and the step caps listed at hcb200_path_stats (the stats limits apply when
+ * d_stats != NULL; hc_max_steps == INT_MAX and hc_max_correction_steps > INT_MAX - 4 always). */
 int hcb200_track(void* stream, int n_hyp,
                  int hc_max_steps, int hc_max_correction_steps, int hc_delta_t_incremental_steps, unsigned flags,
                  const float* d_start_sols, const float* d_start_params,
@@ -105,7 +111,9 @@ int hcb200_track(void* stream, int n_hyp,
  *                                                                                          (d_Trifocal_Sols_Batch_Index)
  *   d_best            optional (may be NULL) hcb200_best_record, written when the launch drains.
  * Paths that start after the flag is up are skipped (converged = 0, end point = start solution) like the reference;
- * unlike the reference the flag is also polled at every HC step, and the infinity flag of skipped paths is 0. */
+ * unlike the reference the flag is also polled at every HC step, and the infinity flag of skipped paths is 0.
+ * Refuses with cudaErrorInvalidValue, nothing launched, what hcb200_track refuses (the step caps of hcb200_path_stats included),
+ * n_edgels outside [1, 65535], or a NULL edgel, K, found or found-index buffer.  hcb200_track_abort_peers refuses the same. */
 int hcb200_track_abort(void* stream, int n_hyp, int n_edgels,
                        int hc_max_steps, int hc_max_correction_steps, int hc_delta_t_incremental_steps, unsigned flags,
                        const float* d_start_sols, const float* d_start_params,
@@ -154,7 +162,8 @@ int hcb200_track_abort_peers(void* stream, int n_hyp, int n_edgels,
  *   flags: HCB200_FLAG_PRUNE_PATHS; the split flag is ignored, as in hcb200_track_abort.
  * Returns cudaErrorInvalidValue, before any CUDA call and with nothing launched, for NULL buffers (d_best and d_stats may be NULL),
  * n_problems outside [1, HCB200_BATCH_MAX_PROBLEMS], n_hyp_per_problem < 0, n_problems * n_hyp_per_problem > 3 441 480 (31-bit path ids),
- * hc_max_correction_steps < 1, off[0] != 0, or a problem with 0 or more than 65 535 edgels.  cudaErrorNotSupported in a compiled-problem
+ * hc_max_correction_steps < 1, the step caps listed at hcb200_path_stats (with d_stats, or INT_MAX caps), off[0] != 0, or a problem with 0
+ * or more than 65 535 edgels.  cudaErrorNotSupported in a compiled-problem
  * library.  The limit on n_problems keeps the staged offsets (16 bytes per problem) in one 64 KB copy. */
 #define HCB200_BATCH_MAX_PROBLEMS 4095
 size_t hcb200_batch_workspace_bytes(int n_problems);

@@ -455,11 +455,13 @@ static void perturb_solution(const hco_variant* v, uint32_t path_key, uint32_t s
   }
 }
 
+typedef struct { float* t0; float* delta_t; uint8_t* accepted; int cap, n; } step_trace;   /* hco_trace_path */
+
 /* ------------------------------------------------------------------------------------------------------------
  * one path: …TrunPaths.cu:80-286 (SURVEY.md App. B), cfg->prune == 0 gives CPUHC_Generic_Solver_Eval_by_Indx.cpp:67-172 */
-void hco_track_path_v(const int* dHdx, const int* dHdt, const hco_c32* start_sol31, const hco_c32* sp,
-                      const hco_c32* tp, const hco_c32* dp, const hco_settings* cfg, const hco_variant* v, uint32_t path_key,
-                      hco_c32* out_track31, uint8_t* out_conv, uint8_t* out_inf, hco_path_stats* st)
+static void track_path(const int* dHdx, const int* dHdt, const hco_c32* start_sol31, const hco_c32* sp,
+                       const hco_c32* tp, const hco_c32* dp, const hco_settings* cfg, const hco_variant* v, uint32_t path_key,
+                       hco_c32* out_track31, uint8_t* out_conv, uint8_t* out_inf, hco_path_stats* st, step_trace* trace)
 {
   const int ltr = v ? v->term_order : 0, contract = v ? v->contract : 0;
   uint32_t solve_no = 0;
@@ -487,6 +489,7 @@ void hco_track_path_v(const int* dHdx, const int* dHdt, const hco_c32* start_sol
     t_step = t0;
     const float half = 0.5f * delta_t;
     s.steps++;
+    if (trace && trace->n < trace->cap) { trace->t0[trace->n] = t0; trace->delta_t[trace->n] = delta_t; trace->accepted[trace->n++] = 0; }
 
     /* RK4 predictor, "loopy" form (:170-211) */
     for (int r = 0; r < 4; r++) {
@@ -551,6 +554,7 @@ void hco_track_path_v(const int* dHdx, const int* dHdt, const hco_c32* start_sol
       counter++;
       for (int i = 0; i < HCO_N; i++) last[i] = sols[i] = x[i];
       if (counter >= cfg->dt_inc_steps) { counter = 0; delta_t *= 2.0f; }
+      if (trace && trace->n == s.steps) trace->accepted[trace->n - 1] = 1;
     }
   }
   const int conv = ((double)t0 >= 1.0 || (1.0 - (double)t0 <= 0.0000001));                           /* :284 */
@@ -559,6 +563,20 @@ void hco_track_path_v(const int* dHdx, const int* dHdt, const hco_c32* start_sol
   *out_conv = (uint8_t)conv;
   *out_inf = (uint8_t)inf_fail;
   if (st) *st = s;
+}
+
+void hco_track_path_v(const int* dHdx, const int* dHdt, const hco_c32* start_sol31, const hco_c32* sp,
+                      const hco_c32* tp, const hco_c32* dp, const hco_settings* cfg, const hco_variant* v, uint32_t path_key,
+                      hco_c32* out_track31, uint8_t* out_conv, uint8_t* out_inf, hco_path_stats* st)
+{ track_path(dHdx, dHdt, start_sol31, sp, tp, dp, cfg, v, path_key, out_track31, out_conv, out_inf, st, NULL); }
+
+int hco_trace_path(const int* dHdx, const int* dHdt, const hco_c32* start_sol31, const hco_c32* sp, const hco_c32* tp, const hco_c32* dp,
+                   const hco_settings* cfg, int cap, float* t0, float* delta_t, uint8_t* accepted,
+                   hco_c32* out_track31, uint8_t* out_conv, uint8_t* out_inf, hco_path_stats* st)
+{
+  step_trace trace = {t0, delta_t, accepted, cap, 0};
+  track_path(dHdx, dHdt, start_sol31, sp, tp, dp, cfg, NULL, 0u, out_track31, out_conv, out_inf, st, &trace);
+  return trace.n;
 }
 
 void hco_track_path(const int* dHdx, const int* dHdt, const hco_c32* start_sol31, const hco_c32* sp,

@@ -106,6 +106,13 @@ void hco_track_batch_v(const int* dHdx, const int* dHdt, const hco_c32* start_so
                        const hco_c32* target, const hco_c32* diff, int n_hyp, const hco_settings* cfg, const hco_variant* v, int n_threads,
                        hco_c32* tracks, uint8_t* converged, uint8_t* infinity, hco_path_stats* stats);
 
+/* one path as hco_track_path, with a per-step trace (test helper): for each of the first `cap` steps the path attempts, t0 at the start of
+ * the step, the delta_t the step uses after the end-zone / 0.95 clamps, and 1 if the step was accepted (0 if rejected or if the step
+ * ended the path at infinity).  Returns the number of steps recorded (min(steps, cap)). */
+int hco_trace_path(const int* dHdx, const int* dHdt, const hco_c32* start_sol31, const hco_c32* start_params34,
+                   const hco_c32* target34, const hco_c32* diff34, const hco_settings* cfg, int cap, float* t0, float* delta_t,
+                   uint8_t* accepted, hco_c32* out_track31, uint8_t* out_converged, uint8_t* out_infinity, hco_path_stats* out_stats);
+
 /* early-abort scoring of one end point: returns 1 if the solution passes (>= 90 % inliers in both view pairs);
  * n21/n31 receive the inlier counts (0 when the imaginary-part gate fails, gate_out tells). */
 int hco_score_solution(const hco_c32* x31, const float* edgel_locations /*[E][6]*/, int n_edgels, const float* K9,

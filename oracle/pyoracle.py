@@ -137,6 +137,19 @@ class Oracle:
                                    n_hyp, ctypes.byref(cfg), var, n_threads or (os.cpu_count() or 1), _vp(tr), _vp(cv), _vp(inf), _vp(st))
         return f2c(tr), cv, inf, st
 
+    def trace_path(self, target34, diff34, track, prune, max_steps=80, max_corr=3, dt_inc=4):
+        """Path `track` (start-solution index) of one hypothesis, with its step control traced.  Returns t0 float32 [S] at the start of each
+        step, delta_t float32 [S] used by the step (after the clamps), accepted bool [S], and the path's stats [5] (as track()), S = steps."""
+        cap = max(max_steps + 1, 0)
+        t0, dt, acc = np.zeros(cap, np.float32), np.zeros(cap, np.float32), np.zeros(cap, np.uint8)
+        tr, cv, inf = np.zeros((self.N + 1, 2), np.float32), ctypes.c_uint8(), ctypes.c_uint8()
+        st = np.zeros(5, np.int32)
+        cfg = Settings(max_steps, max_corr, dt_inc, 1 if prune else 0)
+        n = self.lib.hco_trace_path(_vp(self.hx), _vp(self.ht), _vp(self._ss[track]), _vp(self._sp), _vp(c2f(target34)), _vp(c2f(diff34)),
+                                    ctypes.byref(cfg), cap, _vp(t0), _vp(dt), _vp(acc), _vp(tr), ctypes.byref(cv), ctypes.byref(inf), _vp(st))
+        assert n == st[0]
+        return t0[:n], dt[:n], acc[:n].astype(bool), st
+
     def score(self, x31, locations, K):
         n21, n31, gate = ctypes.c_int(), ctypes.c_int(), ctypes.c_int()
         loc = np.ascontiguousarray(locations, np.float32)

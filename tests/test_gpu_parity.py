@@ -201,26 +201,6 @@ def test_device_refinement_bit_exact_vs_oracle(tracker, oracle, ransac0):
     assert _bit_equal(tr2, tr1)
 
 
-@pytest.mark.parametrize("max_steps,max_corr,dt_inc", [(40, 2, 2), (120, 5, 6), (80, 1, 1), (0, 3, 4)])
-def test_non_default_hc_settings_bit_exact(tracker, oracle, ransac0, max_steps, max_corr, dt_inc):
-    """GPUHC_Max_Steps / GPUHC_Max_Correction_Steps / GPUHC_Num_Of_Steps_to_Increase_Delta_t are run-time arguments of the launch
-    (gpuhc_settings.yaml:9-11); the shipped values are 80 / 3 / 4."""
-    target, diff, _ = oracle.prepare_target_params(5, 1, ransac0["locations"], ransac0["tangents"])
-    saved = (tracker.max_steps, tracker.max_corr, tracker.dt_inc)
-    try:
-        tracker.max_steps, tracker.max_corr, tracker.dt_inc = max_steps, max_corr, dt_inc
-        for prune in (True, False):
-            tr_o, cv_o, inf_o, st_o = oracle.track(target, diff, prune, max_steps=max_steps, max_corr=max_corr, dt_inc=dt_inc)
-            tracker.upload_params(target, diff)
-            tracker.track(1, prune=prune)
-            tr_g, cv_g, inf_g, st_g = tracker.results(1)
-            assert np.array_equal(cv_g, cv_o) and np.array_equal(inf_g, inf_o)
-            assert np.array_equal(st_g[:, :3], st_o[:, :3])
-            assert _bit_equal(tr_g[:, :30], tr_o[:, :30])
-    finally:
-        tracker.max_steps, tracker.max_corr, tracker.dt_inc = saved
-
-
 @pytest.mark.parametrize("prune", [True, False])
 def test_split_long_paths_gives_identical_results(problem, ransac0, prune):
     """HCB200_FLAG_SPLIT_LONG_PATHS parks a path at a step boundary and resumes it on another warp: flags, end points and every counter must
