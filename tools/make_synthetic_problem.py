@@ -34,6 +34,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 NAME = "coupled_quadrics_8x8"
 NAMES = ("coupled_quadrics_8x8", "dense_quadrics_6x6", "mixed_12x12")
 SIZES = {"coupled_quadrics_8x8": (8, 10, 2), "dense_quadrics_6x6": (6, 7, 0), "mixed_12x12": (12, 14, 3)}      # unknowns, parameters, depth unknowns
+# ptxas's register outcome of the two update-predicate forms, per problem (lib/ptxas_hc_tracker_<name>.log): mixed_12x12 spills with &
+BRANCH_FREE_UPDATE = {"coupled_quadrics_8x8": 1, "dense_quadrics_6x6": 1, "mixed_12x12": 0}
 N_SQUARES = {"coupled_quadrics_8x8": 8, "dense_quadrics_6x6": 6, "mixed_12x12": 6}      # equations that are quadratic in their own unknown: 2^k start solutions
 N, NP = 8, 10
 X_PAD, P_PAD = N, NP
@@ -160,6 +162,9 @@ dHdt_Max_Parts: 6
 # leading unknowns that must become positive for a path to be kept (an extension of this repository: the reference's GPU kernels hard-code
 # 8 depths for the trifocal problem, TrunPaths.cu:148-154); 0 switches pruning off
 Num_Of_Depth_Vars: %d
+# elimination-step update predicate of the compiled tracker (an extension of this repository, codegen/gen_eval.py): 1 forms it with & and
+# without a divergent region, 0 with && and a branch; which one ptxas allocates better depends on the problem (DESIGN.md §3)
+HC_Branch_Free_Update: %d
 
 # identity
 problem_name: %s
@@ -175,7 +180,7 @@ Num_Of_GPUs: 1
 Num_Of_Cores: 4
 RANSAC_Dataset: Synthetic
 Abort_RANSAC_by_Good_Sol: false
-""" % (NAME, N, NP, 1 << N_SQUARES[NAME], hx.shape[1], ht.shape[0], SIZES[NAME][2], NAME, NAME.replace("_", " ")))
+""" % (NAME, N, NP, 1 << N_SQUARES[NAME], hx.shape[1], ht.shape[0], SIZES[NAME][2], BRANCH_FREE_UPDATE[NAME], NAME, NAME.replace("_", " ")))
     return hx, ht, sp, sols
 
 

@@ -44,7 +44,7 @@ P_PAD = 33      # parameter index that holds the constant 1    } (defaults: trif
 X_PAD = 30      # variable index that holds the constant 1     }
 WARP = 32
 SPEC = dict(name="trifocal_2op1p_30x30", n_vars=30, n_params=33, n_tracks=312, hx_terms=8, hx_parts=5, ht_terms=16, ht_parts=6,
-            n_depths=8, trifocal=1)
+            n_depths=8, trifocal=1, branch_free_update=1)
 
 
 def configure(spec):
@@ -67,7 +67,8 @@ def read_problem_dir(path):
             cfg[k.strip()] = v.strip().strip('"')
     spec = dict(name=cfg["problem_name"], n_vars=int(cfg["Num_Of_Vars"]), n_params=int(cfg["Num_Of_Params"]), n_tracks=int(cfg["Num_Of_Tracks"]),
                 hx_terms=int(cfg["dHdx_Max_Terms"]), hx_parts=int(cfg["dHdx_Max_Parts"]), ht_terms=int(cfg["dHdt_Max_Terms"]),
-                ht_parts=int(cfg["dHdt_Max_Parts"]), n_depths=int(cfg.get("Num_Of_Depth_Vars", 0)), trifocal=int(cfg["problem_name"] == "trifocal_2op1p_30x30"))
+                ht_parts=int(cfg["dHdt_Max_Parts"]), n_depths=int(cfg.get("Num_Of_Depth_Vars", 0)), trifocal=int(cfg["problem_name"] == "trifocal_2op1p_30x30"),
+                branch_free_update=int(cfg.get("HC_Branch_Free_Update", 1)))
     if spec["trifocal"]:
         spec["n_depths"] = 8
     hx = np.array(open(os.path.join(path, "dHdx_indx.txt")).read().split(), dtype=np.int64)
@@ -644,6 +645,8 @@ def emit(g, path):
     w("#define HCG_TRACKS %d        /* homotopy paths per hypothesis (Num_Of_Tracks) */" % SPEC["n_tracks"])
     w("#define HCG_NUM_DEPTHS %d      /* leading variables that are depths: positive-depth pruning tests them (0: no pruning) */" % SPEC["n_depths"])
     w("#define HCG_TRIFOCAL %d        /* 1: the trifocal relative-pose problem (in-kernel scoring, pose records, target-parameter gather) */" % SPEC["trifocal"])
+    w("#define HCG_BRANCH_FREE_UPDATE %d   /* elimination-step update predicate: 1 with & (no divergent region), 0 with && (settings key HC_Branch_Free_Update) */"
+      % SPEC["branch_free_update"])
     w("")
     w("#endif")
     text = "\n".join(L) + "\n"
